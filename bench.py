@@ -1,13 +1,14 @@
 """Benchmark of the denoise hot path (BASELINE.json metric: TSP-500 graphs/sec, 50-step categorical).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A "step" = one pass of the hot path over one batch: the full 50-step categorical denoise of
 16 TSP-500 (k=50) instances batched block-diagonally in one call (BASELINE config[1]), per GPU.
 Weak scaling: every rank owns its own batch; no collective inside the loop; for N > 1 the final
 heatmaps are all-gathered over NCCL inside the timed region (north_star).
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  --dump-outputs DIR writes the heat map(s) of the last timed step as DIR/heatmap.npy
+(float32; inputs and sampling seeds are fixed, so runs with the same arguments are comparable output for output).
 """
 import argparse
 import json
@@ -176,7 +177,7 @@ def reference_graphs_per_s(budget_s=20.0):
   fit in ~budget_s (at least 1), extrapolated to 50.  Returns (graphs/s, seconds, threads, steps run) or None."""
   sys.path.insert(0, os.path.join(ROOT, "oracle"))
   import make_ref
-  if not make_ref.available() and make_ref.make(verbose=False) is None:
+  if not make_ref.available():
     return None
   import torch
   sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
@@ -322,6 +323,22 @@ def build_workload(cfg, rank):
               graphs=cfg["batch"], node_only=False, gn_segments=1, args=a)
 
 
+DUMP_BYTES = 60 * 10**6   # --dump-outputs budget: under 64 MB with the .npy headers
+
+
+def dump_outputs(out_dir, arrays):
+  """Writes each array as <out_dir>/<name>.npy in float32.  When together they exceed DUMP_BYTES, each one is cut to a
+  fixed, seeded sample of its flattened elements: the same elements for the same arguments, so runs stay comparable."""
+  os.makedirs(out_dir, exist_ok=True)
+  total = sum(np.size(a) * 4 for a in arrays.values())
+  for name, a in arrays.items():
+    a = np.asarray(a, dtype=np.float32)
+    if total > DUMP_BYTES:
+      keep = a.size * DUMP_BYTES // total
+      a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+    np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def algorithmic_bytes_per_step(wl):
   """SURVEY 8(d): sparse / dense TSP 2 L E H 4 = 24 576 E per denoise step (L-1 inter-layer reads + the head's read,
   L writes; layer 0 reads xt instead of a materialised e0); MIS (2L-2) E H 4 (no e0 read, the last layer's e is never
@@ -409,6 +426,8 @@ def run_ours(args, rank, world, local_rank):
   assert np.isfinite(hm).all()
   if categorical:
     assert hm.min() >= 0.0 and hm.max() <= 1.0 + 1e-5
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, {"heatmap": np.stack([g.cpu().numpy() for g in gathered]) if world > 1 else hm})
 
   # ---- the dominant kernel on its own: ONE more batch with per-launch CUDA events on the launching stream (plain
   #      launches: events cannot be recorded inside the captured graph the timed region replays); not part of `value`
@@ -513,7 +532,13 @@ def main():
   ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
   ap.add_argument("--config", default="C2", choices=sorted(CONFIGS), help="BASELINE.json config (default C2 = configs[1], the headline)")
   ap.add_argument("--no-cpu-baseline", dest="no_cpu_baseline", action="store_true")
+  ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                  help="write the heat map(s) of the last timed step as DIR/heatmap.npy")
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error("--steps must be at least 1")
+  if args.dump_outputs and args.impl != "ours":
+    ap.error("--dump-outputs needs --impl ours")
   rank = int(os.environ.get("RANK", "0"))
   world = int(os.environ.get("WORLD_SIZE", "1"))
   local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -29,22 +29,22 @@ def _sha(path):
   return hashlib.sha256(open(path, "rb").read()).hexdigest()
 
 
-def make(verbose=True):
+def make(verbose=True, src=SRC, dst=DST):
   """Returns the destination directory, or None when the reference tree is not mounted (the GPU box)."""
-  if not os.path.isdir(SRC):
-    return DST if os.path.isdir(DST) else None
+  if not os.path.isdir(src):
+    return dst if os.path.isdir(dst) else None
   for rel in FILES:
-    s, d = os.path.join(SRC, rel), os.path.join(DST, rel)
+    s, d = os.path.join(src, rel), os.path.join(dst, rel)
     os.makedirs(os.path.dirname(d), exist_ok=True)
     if not os.path.exists(d) or _sha(s) != _sha(d):
       shutil.copyfile(s, d)
     assert _sha(s) == _sha(d), rel
-  with open(os.path.join(DST, "MANIFEST.sha256"), "w") as f:
+  with open(os.path.join(dst, "MANIFEST.sha256"), "w") as f:
     for rel in FILES:
-      f.write(f"{_sha(os.path.join(DST, rel))}  {rel}\n")
+      f.write(f"{_sha(os.path.join(dst, rel))}  {rel}\n")
   if verbose:
-    print(f"oracle/_ref: {len(FILES)} reference files copied unmodified to {DST}")
-  return DST
+    print(f"oracle/_ref: {len(FILES)} reference files copied unmodified to {dst}")
+  return dst
 
 
 def available():

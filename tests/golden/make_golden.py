@@ -130,6 +130,26 @@ def gen_forward():
   save("fwd_dense_cat", points=ptsd, xt=xtd, t=td, out=out)
 
 
+def gen_ref_copy():
+  """What tests/test_reference_copy.py compares against: the sha256 of every reference file oracle/make_ref.py copies,
+  and the reference GNNEncoder's forward on the instance that test feeds the oracle port."""
+  sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(HERE)), "oracle"))
+  import hashlib
+  import make_ref
+  path = os.path.join(HERE, "ref_sources.sha256")
+  with open(path, "w") as f:
+    for rel in make_ref.FILES:
+      with open(os.path.join(ref_shims.REFERENCE_ROOT, rel), "rb") as src:
+        f.write(f"{hashlib.sha256(src.read()).hexdigest()}  {rel}\n")
+  print(f"wrote {path}")
+  w2 = syn.make_encoder_weights(0, out_channels=2)
+  pts, ei = syn.tsp_sparse_batch(30, 7, 2, seed=5)
+  xt = (syn.initial_noise(ei.shape[1], 3) > 0).astype(np.float32)
+  m = ref_encoder(w2, 2, False)
+  logits = m(torch.from_numpy(pts), torch.tensor([321.0]), torch.from_numpy(xt), torch.from_numpy(ei)).numpy()
+  save("fwd_tsp_cat_k7", points=pts, edge_index=ei, xt=xt, t=np.array([321.0], np.float32), logits=logits)
+
+
 # ------------------------------------------------------------------------------------------
 class Args(object):
   def __init__(self, **kw):
@@ -412,6 +432,8 @@ if __name__ == "__main__":
     gen_schedules()
   if a.only in ("", "forward"):
     gen_forward()
+  if a.only in ("", "ref_copy"):
+    gen_ref_copy()
   if a.only in ("", "traj"):
     gen_trajectories()
   if a.only in ("", "mis_decode"):

@@ -48,6 +48,24 @@ def test_small_workloads_build_on_cpu():
     assert np.all(np.diff(wl["edge_index"][0]) >= 0) or name == "C1"      # sparse TSP lists arrive row-sorted
 
 
+def test_dump_outputs_float32_and_seeded_sample_within_budget(tmp_path, monkeypatch):
+  hm = np.arange(1000, dtype=np.float64) / 1000
+  bench.dump_outputs(str(tmp_path / "full"), {"heatmap": hm})
+  got = np.load(tmp_path / "full" / "heatmap.npy")
+  assert got.dtype == np.float32 and np.array_equal(got, hm.astype(np.float32))
+  monkeypatch.setattr(bench, "DUMP_BYTES", 1000)             # 4000 bytes of output: a quarter survives
+  for run in ("a", "b"):
+    bench.dump_outputs(str(tmp_path / run), {"heatmap": hm})
+  a, b = np.load(tmp_path / "a" / "heatmap.npy"), np.load(tmp_path / "b" / "heatmap.npy")
+  assert a.size == 250 and np.array_equal(a, b) and np.all(np.diff(a) > 0)
+
+
+def test_steps_below_one_is_rejected():
+  r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], stdout=subprocess.PIPE,
+                     stderr=subprocess.STDOUT, text=True, timeout=600)
+  assert r.returncode == 2 and "--steps" in r.stdout
+
+
 def test_gpu_arm_fails_loudly_without_a_gpu():
   import torch
   if torch.cuda.is_available():

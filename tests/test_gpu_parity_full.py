@@ -256,6 +256,27 @@ def test_fused_loop_graph_capture_matches_plain_launches(weights2):
   assert np.array_equal(a1, a4) and np.isfinite(c1).all()
 
 
+def test_bench_dump_outputs_identical_across_runs(tmp_path):
+  """bench.py --dump-outputs: the heat map of the last timed step; a second run with the same arguments writes the
+  same bits, so two builds can be compared output for output."""
+  import json
+  import os
+  import subprocess
+  import sys
+  root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+  dumps = []
+  for run in range(2):
+    d = tmp_path / str(run)
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--config", "B1", "--steps", "2", "--warmup", "1",
+                        "--no-cpu-baseline", "--dump-outputs", str(d)], capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 2
+    dumps.append(np.load(d / "heatmap.npy"))
+  a, b = dumps
+  assert a.dtype == np.float32 and a.shape == (500 * 50,) and np.array_equal(a, b)
+  assert np.isfinite(a).all() and a.min() >= 0 and a.max() <= 1 + 1e-5    # the last step returns probabilities
+
+
 # ------------------------------------------------------------------------------------------------
 # N-GPU sharding on real GPUs (NCCL): per-instance heat maps bitwise equal to the single-GPU answer
 # ------------------------------------------------------------------------------------------------

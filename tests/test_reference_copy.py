@@ -1,15 +1,15 @@
-"""oracle/_ref (the UNMODIFIED reference files that travel to the GPU box for `bench.py --impl reference`):
-byte identity with /root/reference where that is mounted, manifest consistency everywhere, and the copy's own
-GNNEncoder forward against the oracle port on a tiny instance (run in a subprocess: the dependency shims install
-stand-in modules that must not leak into the other tests)."""
+"""oracle/_ref (the UNMODIFIED reference files that travel with a built tree for `bench.py --impl reference`): the recipe
+oracle/make_ref.py copies byte for byte and writes a matching manifest, a copy that is present is the reference as
+pinned by tests/golden/ref_sources.sha256, and the reference GNNEncoder's own forward (tests/golden/fwd_tsp_cat_k7.npz)
+matches the oracle port.  Both fixtures are written by tests/golden/make_golden.py from the unmodified reference."""
 import hashlib
 import os
-import subprocess
 import sys
 
-import pytest
+from conftest import GOLDEN, ROOT, golden, rel_linf
+from difusco_b200 import synthetic as syn
+from oracle import difusco_oracle as orc
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 import make_ref  # noqa: E402
 
@@ -18,58 +18,40 @@ def _sha(path):
   return hashlib.sha256(open(path, "rb").read()).hexdigest()
 
 
-def _have_copy():
-  if os.path.isdir(make_ref.SRC):
-    return make_ref.make(verbose=False) is not None
-  return make_ref.available()
-
-
-def test_ref_copy_is_byte_identical_and_manifest_matches():
-  if not _have_copy():
-    pytest.skip("neither /root/reference nor oracle/_ref present")
-  manifest = {}
-  for line in open(os.path.join(make_ref.DST, "MANIFEST.sha256")):
+def _manifest(path):
+  out = {}
+  for line in open(path):
     h, rel = line.split()
-    manifest[rel] = h
+    out[rel] = h
+  return out
+
+
+def test_ref_copy_is_byte_identical_and_manifest_matches(tmp_path):
+  # the recipe on a stand-in tree with the reference's layout
+  src, dst = tmp_path / "src", tmp_path / "dst"
+  for i, rel in enumerate(make_ref.FILES):
+    (src / rel).parent.mkdir(parents=True, exist_ok=True)
+    (src / rel).write_bytes(f"# stand-in {i} for {rel}\n".encode())
+  assert make_ref.make(verbose=False, src=str(src), dst=str(dst)) == str(dst)
+  manifest = _manifest(dst / "MANIFEST.sha256")
   assert sorted(manifest) == sorted(make_ref.FILES)
   for rel in make_ref.FILES:
-    d = os.path.join(make_ref.DST, rel)
-    assert _sha(d) == manifest[rel], rel
-    s = os.path.join(make_ref.SRC, rel)
-    if os.path.exists(s):
-      assert _sha(s) == manifest[rel], rel   # unmodified
+    assert (dst / rel).read_bytes() == (src / rel).read_bytes(), rel
+    assert _sha(dst / rel) == manifest[rel], rel
+  # the pinned hashes of the reference cover the recipe's files; a copy that is present is unmodified
+  ref = _manifest(os.path.join(GOLDEN, "ref_sources.sha256"))
+  assert sorted(ref) == sorted(make_ref.FILES)
+  if make_ref.available():
+    assert _manifest(os.path.join(make_ref.DST, "MANIFEST.sha256")) == ref
+    for rel in make_ref.FILES:
+      assert _sha(os.path.join(make_ref.DST, rel)) == ref[rel], rel
   # no reference source may enter the history: the directory is git-ignored
   assert "oracle/_ref/" in open(os.path.join(ROOT, ".gitignore")).read()
 
 
-_CHILD = r"""
-import os, sys
-import numpy as np, torch
-ROOT = sys.argv[1]
-sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "oracle")); sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-import ref_shims
-ref_shims.install(os.path.join(ROOT, "oracle", "_ref", "difusco"))
-from models.gnn_encoder import GNNEncoder as RefEncoder          # the reference's own class from the travelling copy
-import difusco_oracle as orc
-from difusco_b200 import synthetic as syn
-torch.manual_seed(0)
-w = syn.make_encoder_weights(0, out_channels=2)
-enc = RefEncoder(12, 256, 2, aggregation="sum", sparse=True, use_activation_checkpoint=False, node_feature_only=False)
-enc.load_state_dict({k: torch.from_numpy(v) for k, v in w.items()})
-enc.eval()
-pts, ei = syn.tsp_sparse_batch(30, 7, 2, seed=5)
-xt = (syn.initial_noise(ei.shape[1], 3) > 0).astype(np.float32)
-with torch.no_grad():
-  ref = enc(torch.from_numpy(pts), torch.tensor([321.0]), torch.from_numpy(xt), torch.from_numpy(ei))
-out = orc.encoder_forward_sparse_tsp(orc.Weights(w), pts, xt, np.array([321.0], np.float32), ei)
-err = float((ref - out).abs().max() / ref.abs().max())
-print("REL_ERR", err)
-assert err < 1e-5, err
-"""
-
-
 def test_ref_copy_forward_matches_oracle_port():
-  if not _have_copy():
-    pytest.skip("neither /root/reference nor oracle/_ref present")
-  r = subprocess.run([sys.executable, "-c", _CHILD, ROOT], stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=600)
-  assert r.returncode == 0 and "REL_ERR" in r.stdout, r.stdout[-2000:]
+  g = golden("fwd_tsp_cat_k7")
+  w = syn.make_encoder_weights(0, out_channels=2)
+  out = orc.encoder_forward_sparse_tsp(orc.Weights(w), g["points"], g["xt"], g["t"], g["edge_index"])
+  err = rel_linf(out.numpy(), g["logits"])
+  assert err < 1e-5, err
